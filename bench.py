@@ -72,8 +72,10 @@ def parse():
     ap.add_argument("--no-graph", action="store_true", help="time eager launches instead of CUDA graphs (profiling)")
     ap.add_argument("--no-flush", action="store_true", help="do not flush L2 between timed steps")
     ap.add_argument("--cpu-procs", type=int, default=16, help="reference arm: Hogwild worker processes (default 16, capped by the host's cores: the fastest count on the 128-vCPU GPU hosts, pinned so that the GPU/CPU ratio does not move with a probe; 0 = probe 8/16/32/64/all and use the fastest)")
-    ap.add_argument("--cpu-impl", default="auto", choices=["auto", "reference", "port"], help="reference arm: the unmodified reference installed under baseline/_ref, or the oracle port")
+    ap.add_argument("--cpu-impl", default="auto", choices=["auto", "reference", "port"], help="reference arm: the unmodified reference installed under oracle/_ref, or the oracle port")
     ap.add_argument("--cpu-batch", type=int, default=1000, help="reference arm: batch per worker (dglke_train's 1000)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="one GPU: after the timed steps, write what the last of them computed to DIR/<name>.npy (see dump_outputs)")
     return ap.parse_args()
 
 
@@ -124,7 +126,7 @@ def run_reference(args):
         "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": {"workload": desc, "batch_per_worker": B, "workers": nproc,
                    "entities": n_ent_cpu, "entities_scaled_down": scaled,
-                   "note": ("the UNMODIFIED reference (baseline/_ref: KEModel.forward -> loss.backward() -> update, dgl stubbed) "
+                   "note": ("the UNMODIFIED reference (oracle/_ref: KEModel.forward -> loss.backward() -> update, dgl stubbed) "
                             if impl == "reference" else "oracle port of the reference's PyTorch step (oracle/kge_oracle.py) ") +
                            "under dglke_train's process model: Hogwild workers on shared-memory tables, 1 thread each; sampling excluded"},
         "cpu_baseline": {"value": eps, "unit": "edges/s", "cores": nproc, "kind": impl,
@@ -207,6 +209,8 @@ def run_ours(args):
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if world != args.gpus and world > 1:
         args.gpus = world
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs writes the outputs of a one-GPU run")
     cpu_base = None
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         cpu_base = cpu_baseline_subprocess(args)
@@ -250,6 +254,39 @@ def run_ours(args):
         # leave without tearing down NCCL / captured graphs / IPC mappings: destroying a process group whose
         # collectives live inside CUDA graphs has been seen to hang at exit
         os._exit(0)
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, log4, tables):
+    """What a caller of the timed step holds after its last call, as out_dir/<name>.npy (float32; row ids float64):
+
+      log                        the step's (pos_loss, neg_loss, loss, regularization)
+      <table>_emb, <table>_state the updated embedding table and its Adagrad state, for table in (entity, relation)
+
+    tables: {table: (emb, state, ids the step read)}.  A table larger than its share of DUMP_BYTES is written as a
+    seeded sample of the rows that step updated (most rows of a large table are never touched), sorted, with their ids
+    in <table>_rows.npy.  The inputs are seeded, so two builds run with the same arguments can be compared file by file."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"log": log4}
+    share = (DUMP_BYTES - 4096) // len(tables)
+    for name, (emb, state, ids) in tables.items():
+        row_bytes = 4 * emb.shape[1] + 4
+        if emb.shape[0] * row_bytes <= share:
+            arrays[name + "_emb"], arrays[name + "_state"] = emb, state
+            continue
+        rows = torch.unique(ids).cpu().numpy()
+        cap = share // (row_bytes + 8)
+        if len(rows) > cap:
+            rows = np.sort(np.random.default_rng(0).choice(rows, cap, replace=False))
+        idx = torch.from_numpy(rows).to(emb.device)
+        arrays[name + "_rows"] = torch.from_numpy(rows.astype(np.float64))
+        arrays[name + "_emb"], arrays[name + "_state"] = emb[idx], state[idx]
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().cpu().numpy())
 
 
 def measure(args, workload, rank, world, local_rank, dev, cpu_base, K_steps, full):
@@ -389,6 +426,10 @@ def measure(args, workload, rank, world, local_rank, dev, cpu_base, K_steps, ful
     else:
         ms_dev = timed(step_dev)
     clocks = clk.stop() if clk else None
+    if full and args.dump_outputs:
+        last = devb[(K - 1) % NB][0]
+        dump_outputs(args.dump_outputs, eng.log4, {"entity": (ent, ent_state, torch.cat([last[0], last[4]])),
+                                                   "relation": (rel, rel_state, last[3])})
 
     # launches per step, counted from one eager step
     prime()

@@ -1,6 +1,6 @@
 """TEST INFRASTRUCTURE ONLY -- times the reference's CPU implementation of the step on the host cores: the UNMODIFIED
-reference's `KEModel.forward -> loss.backward() -> KEModel.update` when its package is installed under baseline/_ref
-(impl="reference"; `__graft_entry__.build()` pip-installs it there from /root/reference, git-ignored), else the CPU oracle
+reference's `KEModel.forward -> loss.backward() -> KEModel.update` when its package is installed under oracle/_ref
+(impl="reference"; `__graft_entry__.build()` installs it there with oracle/ref_install.py), else the CPU oracle
 (oracle/kge_oracle.py, a port of the same PyTorch step; impl="port").  Both run under the reference's own process model:
 `num_proc` forked Hogwild workers sharing the tables through shared memory, one intra-op thread
 each, a barrier before and after (train.py:290-317, train_pytorch.py:255-259).  Sampling is
@@ -18,6 +18,7 @@ import torch.multiprocessing as mp
 
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 import kge_oracle as ko  # noqa: E402
+from ref_install import REF_DIR, installed as reference_installed  # noqa: E402,F401
 
 
 def make_batches(n_ent, n_rel, B, Ns, n_batches, seed):
@@ -34,13 +35,6 @@ def make_batches(n_ent, n_rel, B, Ns, n_batches, seed):
         out.append(dict(node_ids=T(nodes), head_local=T(inv[:B]), tail_local=T(inv[B:]), rel_ids=T(r),
                         neg_ids=T(ng), neg_head=bool(k % 2)))
     return out
-
-
-REF_DIR = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "baseline", "_ref")
-
-
-def reference_installed():
-    return os.path.isdir(os.path.join(REF_DIR, "dglke"))
 
 
 def build_reference_model(hp, n_ent, n_rel):
